@@ -7,6 +7,11 @@
 One "step" = one full train step (H2D of the batch where applicable, forward, backward, gradient all-reduce
 over NCCL for N>1, stabiliser check, fused SGD) of Cube R-CNN DLA34_FPN on a synthetic batch of 32 images
 640x640 per GPU (BASELINE configs[1]; weak scaling: the global batch is 32*N).  Prints ONE JSON line on rank 0.
+
+    python bench.py --steps K --warmup W --dump-outputs DIR      # + what the last timed step computed, as DIR/*.npy
+
+The inputs (model init, synthetic batches) are seeded, so two builds run with the same arguments can be compared output
+for output (see dump_outputs).
 """
 import argparse
 import json
@@ -46,7 +51,14 @@ def parse():
     ap.add_argument("--skip-iou", action="store_true")
     ap.add_argument("--skip-torch-baseline", action="store_true",
                     help="do not time the oracle model in stock PyTorch eager on the GPU (baseline_torch_gpu)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 class ClockSampler:
@@ -393,6 +405,28 @@ def iou_block(peak_hbm, peak_src):
     return out
 
 
+DUMP_SAMPLE = 1 << 23      # parameter positions dumped: 32 MB of float32
+
+
+def dump_outputs(out_dir, model, losses):
+    """What one train step hands its caller: the loss dict (LOSS_KEYS order -> losses.npy) and, through the model, the
+    updated parameters.  Those are ~48 M values, so params_sample.npy holds DUMP_SAMPLE positions of the concatenated
+    model.parameters() (each flattened in its torch layout), drawn with a fixed seed.  Gradients are left out: they are
+    the trainer's scratch (zeroed by every step) and vary far more from run to run than the parameters or losses.
+    Two runs of one build (--steps 10, B200 at 1000 W) differ by up to 3e-4 of max |loss| and 1e-5 of max |param|."""
+    import numpy as np
+    import torch
+    from omni3d_b200.train import LOSS_KEYS
+    flat_p = torch.cat([p.detach().reshape(-1) for p in model.parameters() if p.requires_grad])
+    n = flat_p.numel()
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_SAMPLE), replace=False))
+    out = {"losses": torch.stack([losses[k].detach().float() for k in LOSS_KEYS]),
+           "params_sample": flat_p[torch.from_numpy(idx).to(flat_p.device)]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -432,7 +466,7 @@ def run_ours(args):
         n0 = _lib.LAUNCHES["n"]
         e0.record()
         for i in range(steps):
-            trainer.step(batches[i % 2])
+            losses = trainer.step(batches[i % 2])
             if read_loss:
                 trainer.status(wait=True)          # device->host read of the step's losses (pinned, 56 bytes)
         e1.record()
@@ -444,18 +478,21 @@ def run_ours(args):
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t)
-        return ms, _lib.LAUNCHES["n"] - n0
+        return ms, _lib.LAUNCHES["n"] - n0, losses
 
     for i in range(max(args.warmup, 3)):
         trainer.step(resident[i % 2])
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms, launches = timed(resident, args.steps, read_loss=False)
+    ms, launches, losses = timed(resident, args.steps, read_loss=False)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # before the e2e steps: a replayed CUDA graph rewrites the same loss tensors and parameters in place
+        dump_outputs(args.dump_outputs, model, losses)
     for i in range(2):
         trainer.step(host[i % 2])
-    ms_e2e, _ = timed(host, args.steps, read_loss=True)
+    ms_e2e, _, _ = timed(host, args.steps, read_loss=True)
     status = trainer.status()
     peak_tf, peak_hbm, peak_src = peaks()
     # the instrumented step runs on EVERY rank (it contains the same collectives as any other step)

@@ -18,6 +18,7 @@ CASES = {"dla34": ("configs/cubercnn_DLA34_FPN.yaml", (128, 160)), "resnet34": (
 
 
 def main():
+    torch.set_num_threads(8)        # = FIXTURE_THREADS of tests/test_model_oracle.py (results depend on the thread count)
     out = {}
     for name, (cfg_file, (H, W)) in CASES.items():
         cfg = ref_runner.reference_cfg(cfg_file)

@@ -451,6 +451,39 @@ int32_t c3d_resize_bilinear_u8(const uint8_t* img_hwc, int32_t H, int32_t W, int
                                int32_t ksize_v, int32_t new_h, int32_t new_w, int32_t row_first, int32_t row_last,
                                int32_t flip, uint8_t* tmp_hwc, uint8_t* out_chw, void* stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Omni3D AP evaluation (omni3d_b200/csrc/eval_ops.cu): Omni3Deval.evaluate / accumulate of
+ * cubercnn/evaluation/omni3d_evaluation.py:1172-1313, 1315-1357, 1433-1551 for every (image, category) group at once.
+ * ------------------------------------------------------------------------------------------ */
+/* Greedy matching, replacing the per-(category, range, image) evaluateImg calls (:1347-1352, loop :1489-1536).
+ * Groups are back to back: group g owns detections [dt_off[g], dt_off[g+1]) — already sorted by -score (stable) and
+ * truncated to maxDets[-1] — and ground truths [gt_off[g], gt_off[g+1]) in annotation order (int32 [num_groups+1]).
+ *   dt_box / gt_box [n][4] fp64 XYWH; dt_rng / gt_rng [n] fp64 = area (2D) or depth (3D); gt_ignore [n_gt] (0/1);
+ *   gt_id [n_gt] int64 annotation ids.  mode3d != 0: IoU = (double) iou3d[pair_off[g] + d * ng + j], the packed fp32
+ *   matrices of c3d_box3d_overlap_segmented over the same groups; else pycocotools bbIou (iscrowd 0) in fp64.
+ *   eval_prox != 0: a GT is a candidate only if bbIou(dt, gt) > prox_thresh, a detection with no such GT is ignored.
+ *   iou_start_host [T] = min(iouThrs[t], 1 - 1e-10); ranges_host [A][2] = inclusive bounds (HOST arrays; A <= 8, T <= 16).
+ * Outputs, chain c = a * T + t:  match [A*T][n_dt] int32 = matched GT row (global index) or -1;
+ *   flags [A*T][n_dt] uint8 = bit 0 dtIgnore, bit 1 dtMatches != 0 (the matched GT's id is non-zero);
+ *   npig [num_groups][A] int32 = number of non-ignored GTs.  Workspace: c3d_eval_match_workspace_bytes(n_gt, A, T). */
+size_t c3d_eval_match_workspace_bytes(int64_t n_gt, int32_t A, int32_t T);
+int32_t c3d_eval_match(int32_t mode3d, int32_t eval_prox, int32_t num_groups, int32_t A, int32_t T,
+                       const int32_t* dt_off, const int32_t* gt_off, const double* dt_box, const double* dt_rng,
+                       const double* gt_box, const double* gt_rng, const uint8_t* gt_ignore, const int64_t* gt_id,
+                       const float* iou3d, const int64_t* pair_off, int64_t n_dt, int64_t n_gt,
+                       const double* iou_start_host, const double* ranges_host, double prox_thresh, int32_t* match,
+                       uint8_t* flags, int32_t* npig, void* workspace, size_t workspace_bytes, void* stream);
+/* Precision / recall / score tables, replacing the (category, range, maxDet, threshold) loops of accumulate (:1227-1299).
+ * Category k sums npig over the groups [grp_off[k], grp_off[k+1]) (rows of npig [.][A]) and owns the entries
+ * [ent_off[k], ent_off[k+1]) (int32 [K+1]), sorted by -score (stable over image order, then per-group rank): entry e is
+ * column ent_idx[e] of flags [A*T][n_dt] (as c3d_eval_match writes it), with per-group rank ent_rank[e] and score
+ * ent_score[e] (fp64).  rec_thrs [R] fp64 and max_dets [M] int32 are device arrays; T * M <= 64.
+ * precision / scores [T][R][K][A][M] and recall [T][K][A][M] (fp64) are written in full, -1 where npig == 0.  No workspace. */
+int32_t c3d_eval_accumulate(int32_t K, int32_t A, int32_t T, int32_t M, int32_t R, const int32_t* grp_off,
+                            const int32_t* npig, const int32_t* ent_off, const int32_t* ent_idx, const int32_t* ent_rank,
+                            const double* ent_score, const uint8_t* flags, int64_t n_dt, const double* rec_thrs,
+                            const int32_t* max_dets, double* precision, double* recall, double* scores, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -66,4 +66,5 @@ EXPORTS = [
     "c3d_topk_segments", "c3d_label_sample_proposals", "c3d_anchor_sample_keys", "c3d_anchor_sample_finish", "c3d_det_candidates",
     "c3d_box_loss_fwd", "c3d_box_loss_bwd", "c3d_cube_gather", "c3d_cube_reduce_fwd", "c3d_cube_reduce_bwd", "c3d_cube_scatter",
     "c3d_linear_fwd_blocks", "c3d_linear_dgrad_blocks", "c3d_linear_wgrad_blocks", "c3d_resize_bilinear_u8", "c3d_preprocess_batch", "c3d_pack_conv_weights_batched",
+    "c3d_eval_match_workspace_bytes", "c3d_eval_match", "c3d_eval_accumulate",
 ]
